@@ -1,7 +1,8 @@
 #!/usr/bin/env python
-"""bench.py — the driver's benchmark contract for the simpledet_b200 hot path.
+"""bench.py — the benchmark of the simpledet_b200 hot path.
 
-  python bench.py --gpus N --steps K --warmup W            (our CUDA path)
+  python bench.py --gpus N --steps K --warmup W            (our CUDA path; K timed steps)
+  python bench.py ... --dump-outputs DIR                   (also writes the last timed step's outputs as .npy)
   python bench.py --impl reference --gpus N --steps K ...  (the reference's CPU path = oracle)
   python bench.py --workload retina_train|mask_train|dcn_softnms ...   (BASELINE.json configs 3-5)
 
@@ -22,6 +23,7 @@ north-star shape 512 rois x 256 ch x 14x14 timed in the same process.
 from __future__ import annotations
 
 import argparse
+import gc
 import json
 import os
 import subprocess
@@ -38,7 +40,6 @@ STRIDES_ROI = (4, 8, 16, 32)
 IMG_H, IMG_W = 800, 1333
 C_FEAT, N_ROI, K_CLS, POOLED = 256, 1000, 81, 7
 GRAD_BUCKET_FLOATS = 41_500_000  # ~41.5 M parameters of faster_r50v1_fpn -> 166 MB fp32 (SURVEY §8e)
-MIN_TIMED_SECONDS = 0.5          # the K-step block is repeated until the timed region is at least this long
 
 
 def level_shapes(strides):
@@ -92,8 +93,9 @@ class Infer:
         # (RoI head: 2 fc + cls/reg fc on tensor cores — library GEMMs, not on this path)
         bbox = ops.DecodeBBox(rois, d["head_bbox_pred"], d["im_info"], (0, 0, 0, 0), (0.1, 0.1, 0.2, 0.2),
                               class_agnostic=False)
-        dets, counts, keep, nkeep, _ = ops.multiclass_nms(d["cls_score"], bbox, 0.5, 0.05, first_class=1)
-        return {"rois": rois, "result": (dets, counts, keep, nkeep)}
+        dets, counts, keep, nkeep, src = ops.multiclass_nms(d["cls_score"], bbox, 0.5, 0.05, first_class=1)
+        return {"rois": rois, "result": (dets, counts, keep, nkeep),
+                "outputs": {"rois": rois, "decoded_bbox": bbox, **nms_outputs(dets, counts, keep, nkeep, src)}}
 
     @staticmethod
     def roofline_bytes(out, d, B):
@@ -177,7 +179,8 @@ class RetinaTrain:
         if ev:
             ev[1].record()
         bl = d["bbox_loss"].detach().requires_grad_(True)
-        ops.BBoxNorm(bl, d["reg_label"]).backward(d["bbox_loss"])
+        bn = ops.BBoxNorm(bl, d["reg_label"])
+        bn.backward(d["bbox_loss"])
         scales = tuple(4 * 2 ** (i / 3) for i in range(3))
         boxes, scores = [], []
         for s in cls.STRIDES:
@@ -188,8 +191,11 @@ class RetinaTrain:
             boxes.append(b_)
             scores.append(s_)
         boxes, scores = torch.cat(boxes, 1), torch.cat(scores, 1)
-        dets, counts, keep, nkeep, _ = ops.multiclass_nms(scores, boxes, 0.5, 0.05, first_class=1)
-        return {"result": (logits.grad[:, :1024, :].contiguous(), bl.grad[:, :, :256].contiguous(), nkeep)}
+        dets, counts, keep, nkeep, src = ops.multiclass_nms(scores, boxes, 0.5, 0.05, first_class=1)
+        return {"result": (logits.grad[:, :1024, :].contiguous(), bl.grad[:, :, :256].contiguous(), nkeep),
+                "outputs": {"focal_prob": out, "focal_grad": logits.grad, "bbox_norm": bn, "bbox_norm_grad": bl.grad,
+                            "retina_boxes": boxes, "retina_scores": scores,
+                            **nms_outputs(dets, counts, keep, nkeep, src)}}
 
     @classmethod
     def roofline_bytes(cls, out, d, B):
@@ -260,7 +266,11 @@ class MaskTrain:
         ml = d["mask_logit"].detach().requires_grad_(True)
         loss = ops.SigmoidCrossEntropy(ml, mask_t.reshape(B * 128, 28 * 28))
         loss.backward(loss.new_ones(loss.shape))
-        return {"rois": rois512, "result": (loss, feats[3].grad, ml.grad[:64].contiguous())}
+        names = ("rois", "label", "bbox_target", "bbox_weight", "mask_target")
+        return {"rois": rois512, "result": (loss, feats[3].grad, ml.grad[:64].contiguous()),
+                "outputs": {**{"target_" + n: t for n, t in zip(names, r)}, "roi_feat7": o7, "roi_feat14": o14,
+                            **{f"feat{s}_grad": f.grad for s, f in zip(STRIDES_ROI, feats)},
+                            "mask_loss": loss, "mask_logit_grad": ml.grad}}
 
     @staticmethod
     def roofline_bytes(out, d, B):
@@ -334,7 +344,8 @@ class DcnSoftNms:
                 ev[1].record()
             x = torch.matmul(col_t, wp).view(B, H, W, C)   # dense contraction: cuBLAS (library work); output channels-last
         ob, oi, oc = ops.soft_nms_batched(d["dets"], 0.5, 0.5, 0.001, 1, counts=d["counts"])
-        return {"result": (x[..., :8].contiguous(), oc)}
+        return {"result": (x[..., :8].contiguous(), oc),
+                "outputs": {"dcn_out": x, "soft_nms_boxes": (ob, oc), "soft_nms_inds": (oi, oc), "soft_nms_counts": oc}}
 
     @staticmethod
     def roofline_bytes(out, d, B):
@@ -363,6 +374,37 @@ class DcnSoftNms:
 
 
 WORKLOADS = {w.name: w for w in (Infer, RetinaTrain, MaskTrain, DcnSoftNms)}
+DUMP_SAMPLE = 1 << 20  # --dump-outputs: larger outputs are written as this many elements at fixed, seeded positions
+
+
+def nms_outputs(dets, counts, keep, nkeep, src):
+    """multiclass_nms's arrays; a (tensor, counts) pair marks rows past counts[p] of problem p as unspecified."""
+    return {"nms_dets": (dets, counts), "nms_counts": counts, "nms_keep": (keep, nkeep), "nms_nkeep": nkeep,
+            "nms_src": (src, counts)}
+
+
+def dump_outputs(outputs, out_dir):
+    """Write each output of a step as out_dir/<name>.npy: floating point as float32, integers as float64 (exact).
+    Rows an operator leaves unspecified are written as 0; an output of more than DUMP_SAMPLE elements is written as
+    the elements at DUMP_SAMPLE flat positions drawn with a fixed seed, in increasing order."""
+    import torch
+
+    os.makedirs(out_dir, exist_ok=True)
+    total = 0
+    for name, x in outputs.items():
+        if isinstance(x, tuple):
+            x, n = x
+            valid = torch.arange(x.shape[1], device=x.device)[None, :] < n.reshape(-1, 1).to(x.device)
+            x = torch.where(valid.reshape(valid.shape + (1,) * (x.dim() - 2)), x, torch.zeros((), dtype=x.dtype,
+                                                                                               device=x.device))
+        x = x.detach()
+        if x.numel() > DUMP_SAMPLE:
+            idx = np.sort(np.random.default_rng(0).choice(x.numel(), DUMP_SAMPLE, replace=False))
+            x = x.reshape(-1)[torch.from_numpy(idx).to(x.device)]
+        a = x.cpu().numpy().astype(np.float32 if x.is_floating_point() else np.float64)
+        total += a.nbytes
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+    assert total <= 64 << 20, f"--dump-outputs wrote {total} bytes"
 
 
 def roialign_algorithmic_bytes(rois_np, B, pooled, with_argmax, n_roi=None, C=C_FEAT):
@@ -580,34 +622,29 @@ def run_ours(args):
     # ---- device-resident throughput (`value`) ----
     for i in range(W):
         out = one_step(dev_sets[i % R])
-    sync_all()
-    # repeat the K-step block until the timed region is long enough for the clock sampler to see load
-    e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-    e0.record()
-    for i in range(K):
-        one_step(dev_sets[i % R])
-    e1.record()
-    torch.cuda.synchronize()
-    reps = max(1, int(np.ceil(MIN_TIMED_SECONDS / max(e0.elapsed_time(e1) / 1e3, 1e-6))))
-    if world > 1:
-        t = torch.tensor([reps], device=dev)
-        dist.all_reduce(t, op=dist.ReduceOp.MAX)
-        reps = int(t.item())
     ar_events.clear()
+    e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     kev = [(torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)) for _ in range(K)]
     sync_all()
     n0 = _lib.launch_count()
+    gc.disable()  # as timeit does: a collector pass landing in some windows of K steps and not in others is noise
     with ClockSampler(local) as clk:
         e0.record()
-        for r_ in range(reps):
-            for i in range(K):
-                one_step(dev_sets[i % R], kev[i] if r_ == reps - 1 else None)
+        # only the final step's outputs are kept: holding each step's into the next would make the caching
+        # allocator grow (cudaMalloc) inside the timed region
+        for i in range(K - 1):
+            one_step(dev_sets[i % R], kev[i])
+        last = one_step(dev_sets[(K - 1) % R], kev[K - 1])
         e1.record()
         sync_all()
-    launches = (_lib.launch_count() - n0) // reps
-    ms = shard.max_over_ranks(e0.elapsed_time(e1), dev) / reps
+    gc.enable()
+    launches = _lib.launch_count() - n0
+    ms = shard.max_over_ranks(e0.elapsed_time(e1), dev)
     k_us = float(np.mean([a.elapsed_time(b) for a, b in kev])) * 1e3
     ar_ms = float(np.median([a.elapsed_time(b) for a, b in ar_events])) if ar_events else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(last["outputs"], args.dump_outputs)
+    del last
 
     # ---- end to end through the public API with HOST buffers (`e2e`) ----
     # Every step copies its inputs from pinned host memory and reads its result back into pinned host memory; all
@@ -658,23 +695,13 @@ def run_ours(args):
     res = e2e_run(3)
     d2h_bytes = sum(x.numel() * x.element_size() for x in res)
     sync_all()
-    e0.record()
-    e2e_run(K)
-    e1.record()
-    torch.cuda.synchronize()
-    ereps = max(1, int(np.ceil(MIN_TIMED_SECONDS / max(e0.elapsed_time(e1) / 1e3, 1e-6))))
-    if world > 1:
-        t = torch.tensor([ereps], device=dev)
-        dist.all_reduce(t, op=dist.ReduceOp.MAX)
-        ereps = int(t.item())
-    sync_all()
     with ClockSampler(local) as clk2:
         e0.record()
-        e2e_run(K * ereps)
+        e2e_run(K)
         e1.record()
         sync_all()
     clk.rows += clk2.rows  # clocks are reported over both timed regions
-    e2e_local = e0.elapsed_time(e1) / ereps
+    e2e_local = e0.elapsed_time(e1)
     e2e_ms = shard.max_over_ranks(e2e_local, dev)
     h2d_gbs = h2d_bytes * K / (e2e_local * 1e-3) / 1e9
     if world > 1:
@@ -745,7 +772,7 @@ def run_ours(args):
                    "parallelism": f"dp{world} (sharded by image" + (", one fp32 gradient all-reduce per step)" if wl.train
                                                                       else ", no data-path collective)"),
                    "l2": f"{R} rotating input sets ({int(R * set_mb)} MB) larger than L2, no flush",
-                   "timed_region": f"{reps} x {K} steps (>= {MIN_TIMED_SECONDS} s), e2e {ereps} x {K}",
+                   "timed_region": f"{K} steps, e2e {K} steps",
                    "numa_binding": numa, "weights": "random synthetic activations (seeded)"},
         "clocks": clk.summary(),
         "e2e": {"value": round(e2e_value, 2), "unit": "images/s", "h2d_bytes_per_step": h2d_bytes,
@@ -800,6 +827,9 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-target", action="store_true", help="skip the north-star-shape measurement (keeps an ncu launch "
                     "list of the step free of its launches)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step computed as DIR/<name>.npy "
+                    "(float32, integers as float64; outputs over %d elements as a fixed seeded sample), so that two "
+                    "builds can be compared on identical inputs" % DUMP_SAMPLE)
     args = ap.parse_args()
     if args.impl == "reference":
         run_reference(args)
