@@ -110,8 +110,11 @@ def test_fpn_bench_shape_small_c_cl(cuda):
 
 
 def test_fpn_target_shape_full_cl(cuda):
-    _fpn(1, 512, 256, 14, cuda, 0, False)
+    """The north-star shape, all 256 channels, bit for bit against the oracle's literal 4-level graph."""
+    _fpn(1, 512, 256, 14, cuda, 0, True)
 
 
 def test_fpn_bench_shape_full_cl(cuda):
-    _fpn(2, 1000, 256, 7, cuda, 1, False)
+    """roi_align_cl_kernel<256, 2>, the kernel of the headline metric, at the bench shape: all 256 channels against
+    the oracle."""
+    _fpn(2, 1000, 256, 7, cuda, 1, True)

@@ -165,6 +165,29 @@ def test_headline_shape_properties(cuda):
     assert ((ax == -1) == (ay == -1)).all()
 
 
+@pytest.mark.parametrize("pooled,n", [(7, 512), (14, 128)])
+def test_training_forward_full_channels_with_argmax(cuda, pooled, n):
+    """The training forward (argmax planes) at mask_train's shapes: B=2, 256 channels on the 800x1333 pyramid,
+    512 rois per image at 7x7 and 128 at 14x14.  out, argmax_x and argmax_y bit for bit against the oracle, run once
+    per level on the rois assigned to it (equivalent to the literal graph: test_fpn_fused_equals_reference_graph)."""
+    rng = np.random.default_rng(19 + pooled)
+    rois = synth.random_rois(rng, 2, n)
+    feats = [rng.standard_normal((2, 256, h, w)).astype(np.float32) for h, w in synth.fpn_shapes()]
+    out, ax, ay, lv = ops.fpn_roi_align_raw([_t(f, cuda) for f in feats], _t(rois, cuda), synth.FPN_STRIDES, pooled)
+    idx = oracle.fpn_assign_levels(rois, synth.FPN_STRIDES).reshape(2, n)
+    assert np.array_equal(lv.cpu().numpy(), idx)
+    assert set(np.unique(idx)) == {0, 1, 2, 3}, "every level must receive rois"
+    o, x, y = out.cpu().numpy(), ax.cpu().numpy(), ay.cpu().numpy()
+    for b in range(2):
+        for i, s in enumerate(synth.FPN_STRIDES):
+            m = idx[b] == i
+            if not m.any():
+                continue
+            ro, rx, ry = oracle.roi_align_v2_forward(feats[i][b:b + 1], rois[b:b + 1, m], (pooled, pooled), 1.0 / s)
+            assert np.array_equal(o[b, m], ro[0]), f"out differs on image {b}, level {i}"
+            assert np.array_equal(x[b, m], rx[0]) and np.array_equal(y[b, m], ry[0]), f"argmax, image {b} level {i}"
+
+
 def test_error_codes(cuda):
     from simpledet_b200._lib import SdetError
 

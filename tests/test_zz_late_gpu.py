@@ -1,9 +1,6 @@
-"""GPU twins of the operators added after this round's 180 GPU-minutes were spent (round 2, last session): they
-could not be run on a B200 by the builder, so the driver's round-end run is their FIRST run on a device.  Their host
-logic and, for kernels, the kernel source itself run on the CPU in tests/test_bbox_target_host.py and
-tests/test_mask_paste_host.py.  They are marked xfail(strict=False) for exactly that reason and nothing else: an
-XPASS in the driver's record is the device confirmation, an XFAIL is a defect of these late additions that must not
-mask the 200+ device-verified tests before them (the file sorts last for the same reason)."""
+"""GPU twins of the operators added last: the device side of bbox_target, the test-time mask paste and the other
+late additions.  Their host logic and, for kernels, the kernel source itself also run on the CPU in
+tests/test_bbox_target_host.py and tests/test_mask_paste_host.py."""
 import os
 
 import numpy as np
@@ -12,9 +9,7 @@ import torch
 
 from simpledet_b200 import ops
 
-pytestmark = [pytest.mark.gpu,
-              pytest.mark.xfail(strict=False, reason="written after the round's GPU budget was spent; first device run "
-                                                     "is the driver's (see the module docstring)")]
+pytestmark = pytest.mark.gpu
 GOLD = os.path.join(os.path.dirname(__file__), "golden")
 
 
